@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # our CUDA path
   python bench.py --impl reference --gpus N --steps K ...   # CPU arm (oracle port of the jxl-rs CPU path)
+  python bench.py --gpus 1 --steps K --dump-outputs DIR     # also write the last step's pixels, to compare two builds
 
 A "step" decodes one batch of synthetic VarDCT frames. Default = BASELINE config 2: 64 frames of 3840x2160 per GPU,
 seeds 2000 + rank*frames + i, 1.19 bits per pixel of file (0.94 of them HF sections), mixed transforms, Gaborish on,
@@ -52,7 +53,14 @@ def parse_args():
     ap.add_argument("--inflight", type=int, default=5, help="resident batches alternated by the device-resident loop")
     ap.add_argument("--e2e-depth", type=int, default=5, help="contexts (batches in flight) of the end-to-end leg's PipelinedDecoder")
     ap.add_argument("--chunk", type=int, default=16, help="frames per chunk of the pipelined end-to-end decode")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the pixels the last step decoded (rank 0; a fixed, seeded sample of "
+                         "pixel positions, the same in every frame) as float32 DIR/<name>.npy, under 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's outputs; --impl reference keeps none")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     cfg = {2: (64, 3840, 2160, 2), 3: (max(1, 512 // world), 1920, 1080, 2), 4: (1, 16384, 16384, 3), 5: (8, 4096, 4096, 0)}[args.config]
     args.frames = cfg[0] if args.frames is None else args.frames
@@ -198,6 +206,36 @@ def cpu_sample_size(args, cores):
     return max(1, min(args.frames, max(args.cpu_sample_frames, cores)))
 
 
+DUMP_BYTES = 20 << 20  # per dumped array: two arrays and their pixel index stay under 64 MB
+
+
+def sample_index(height, width, frames):
+    """Row-major pixel positions that --dump-outputs keeps of every frame: all of them when they fit DUMP_BYTES, else a
+    sorted sample drawn with a fixed seed, so that every run and every build of the project keeps the same ones."""
+    import numpy as np
+    k = min(height * width, DUMP_BYTES // (frames * 3 * 4))
+    return np.sort(np.random.default_rng(0).choice(height * width, k, replace=False))
+
+
+def output_sample(outs):
+    """float32 (frames, samples, 3): the pixels at sample_index() of one step's H x W x 3 output tensors."""
+    import numpy as np
+    import torch
+    h, w, _ = outs[0].shape
+    idx = torch.from_numpy(sample_index(h, w, len(outs))).to(outs[0].device)
+    return np.stack([o.reshape(-1, 3)[idx].cpu().numpy() for o in outs]).astype(np.float32)
+
+
+def write_outputs(out_dir, samples, height, width):
+    """samples: name -> output_sample() array; written as out_dir/<name>.npy next to out_dir/pixel_index.npy."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    frames = len(next(iter(samples.values())))
+    np.save(os.path.join(out_dir, "pixel_index.npy"), sample_index(height, width, frames).astype(np.float64))
+    for name, a in samples.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def workload_text(args, n):
     return (f"batch of {n} synthetic {args.width}x{args.height} VarDCT frames per GPU (BASELINE config {args.config}), "
             f"distance {args.distance}, transform profile {args.profile}, Gaborish on, EPF iters {args.epf}, RGB u8 out")
@@ -314,6 +352,7 @@ def run_modular(args, rank, world, local_rank, numa):
     clocks = sampler.stop()
     launches = b.stats()["kernel_launches"]
     b.close()
+    dumps = {"device_rgb": output_sample(dev_out)} if args.dump_outputs and rank == 0 else None
     barrier()
     # end to end: bytes -> parse -> batch -> pixels in pinned host memory
     host_out = [torch.empty((H, W, 3), dtype=torch.uint8).pin_memory() for _ in range(n)]
@@ -343,6 +382,9 @@ def run_modular(args, rank, world, local_rank, numa):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     dev_ms_max, e2e_sec_max = float(t[0].item()), float(t[1].item())
     ctx.close()
+    if dumps is not None:
+        dumps["e2e_rgb"] = output_sample(host_out)
+        write_outputs(args.dump_outputs, dumps, H, W)
     if rank == 0:
         peaks = {}
         try:
@@ -493,6 +535,7 @@ def main():
         b.close()
     for c in ctxs[1:]:
         c.close()
+    dumps = {"device_rgb": output_sample(dev_out[(args.steps - 1) % depth])} if args.dump_outputs and rank == 0 else None
     del dev_out
 
     # ---------------- end to end through the public API (host bytes -> host pixels) ----------------
@@ -562,6 +605,10 @@ def main():
         except Exception as e:  # noqa: BLE001
             e2e_err = e2e_err or e
     e2e_ok = not any_failed and e2e_sec_max > 0
+    if dumps is not None:
+        if e2e_ok:
+            dumps["e2e_rgb"] = output_sample(host_out[(args.steps - 1) % e2e_depth])
+        write_outputs(args.dump_outputs, dumps, args.height, args.width)
 
     if rank == 0:
         peaks = {}

@@ -1,4 +1,7 @@
 """Fake device layer for dry runs of bench.py on the CPU (tests/test_bench_dry_run.py and its two-rank driver)."""
+import ctypes
+
+
 class _FakeEvent:
     def __init__(self, enable_timing=False):
         pass
@@ -47,14 +50,23 @@ def install(setattr_fn, fail_e2e=False, gloo=False):
             pass
 
     class FakeBatch:
+        """Every run fills the batch's outputs with its running count (runs: n, reruns: 100 + n), so that a dump shows
+        which step wrote it."""
         runs = 0
+        reruns = 0
 
         def __init__(self, ctx, n=0, staging_threads=0):
             self.n = 0
+            self.outs = []
 
         def add(self, fr, ptr, stride, fmt, out_is_device):
             assert fr.width > 0 and ptr != 0 and stride >= fr.width * 3
             self.n += 1
+            self.outs.append((ptr, stride * fr.height))
+
+        def _fill(self, value):
+            for ptr, nbytes in self.outs:
+                ctypes.memset(ptr, value & 0xff, nbytes)
 
         def set_profile(self, on):
             pass
@@ -63,9 +75,11 @@ def install(setattr_fn, fail_e2e=False, gloo=False):
             FakeBatch.runs += 1
             if fail_e2e and FakeBatch.runs > 6:  # the device-resident leg runs --inflight (5) batches once; later runs belong to the end-to-end leg
                 raise RuntimeError("injected failure of the end-to-end leg")
+            self._fill(FakeBatch.runs)
 
         def rerun_device(self, stream_ptr=0):
-            pass
+            FakeBatch.reruns += 1
+            self._fill(100 + FakeBatch.reruns)
 
         def wait(self):
             pass

@@ -13,10 +13,13 @@ from tests import bench_fakes
 
 
 @pytest.mark.parametrize("fail_e2e", [False, True])
-def test_bench_main_control_flow(monkeypatch, capsys, fail_e2e):
+def test_bench_main_control_flow(monkeypatch, capsys, tmp_path, fail_e2e):
+    import numpy as np
+    import jxl_rs_b200 as j
     bench = bench_fakes.install(monkeypatch.setattr, fail_e2e)
     monkeypatch.setattr(sys, "argv", ["bench.py", "--gpus", "1", "--steps", "3", "--warmup", "3", "--frames", "3",
-                                      "--width", "320", "--height", "200", "--cpu-sample-frames", "1", "--lf-tree", "1"])
+                                      "--width", "320", "--height", "200", "--cpu-sample-frames", "1", "--lf-tree", "1",
+                                      "--dump-outputs", str(tmp_path)])
     for k in ("RANK", "LOCAL_RANK", "WORLD_SIZE"):
         monkeypatch.delenv(k, raising=False)
     bench.main()
@@ -36,6 +39,29 @@ def test_bench_main_control_flow(monkeypatch, capsys, fail_e2e):
         assert line["value"] > 0  # the device-resident measurement survives
     else:
         assert line["e2e"]["value"] > 0 and line["e2e"]["h2d_bytes_per_step"] == 1000
+    # device-resident reruns: 3 warm-up, 1 single-batch stage timing, then exactly --steps timed ones
+    assert j.Batch.reruns == 3 + 1 + 3
+    # 3 frames of 320x200 fit the dump whole; the device-resident pixels are those of the last timed step
+    idx, dev = np.load(tmp_path / "pixel_index.npy"), np.load(tmp_path / "device_rgb.npy")
+    assert idx.dtype == np.float64 and np.array_equal(idx, np.arange(320 * 200))
+    assert dev.dtype == np.float32 and dev.shape == (3, 320 * 200, 3) and (dev == 100 + j.Batch.reruns).all()
+    if fail_e2e:
+        assert not (tmp_path / "e2e_rgb.npy").exists()
+    else:
+        e2e = np.load(tmp_path / "e2e_rgb.npy")
+        assert e2e.dtype == np.float32 and e2e.shape == dev.shape and (e2e == j.Batch.runs).all()
+
+
+def test_dump_sample_is_fixed_and_bounded():
+    """--dump-outputs keeps the same pixel positions in every run and stays under 64 MB (both dumped arrays and the
+    index) in every BASELINE configuration."""
+    import numpy as np
+    import bench
+    for frames, w, h in ((64, 3840, 2160), (512, 1920, 1080), (1, 16384, 16384), (8, 4096, 4096)):
+        idx = bench.sample_index(h, w, frames)
+        assert 2 * frames * len(idx) * 3 * 4 + 8 * len(idx) < 64_000_000
+        assert len(np.unique(idx)) == len(idx) and 0 <= idx[0] and idx[-1] < w * h
+        assert np.array_equal(idx, bench.sample_index(h, w, frames))
 
 
 def test_bench_two_ranks_over_gloo(tmp_path):
