@@ -152,11 +152,6 @@ typedef struct JxgFrameDesc {
  * threads and pinned allocations to the GPU's NUMA node before jxg_init. buf: >= 16 bytes. */
 int jxg_device_pci_bus_id(int device, char* buf, int len);
 
-/* The device's two optional stage streams (JXG_STAGE_STREAMS=1: block plan + entropy decode of every batch on the first,
- * transforms + filters + stores on the second). Off by default - every batch runs on its context's own stream, which
- * measured faster (DESIGN.md section 3); returned so that a host that turns them on can record events on them. */
-int jxg_device_streams(int device, void** entropy_stream, void** post_stream);
-
 /* Context: one per device/rank. Owns streams, pinned staging and device pools. */
 int jxg_init(int device, void** ctx);
 void jxg_shutdown(void* ctx);
@@ -186,7 +181,9 @@ int jxg_batch_rerun_device(void* batch, void* cuda_stream);
 void jxg_batch_end(void* batch);
 
 /* Parity taps: copy intermediate planes of frame `f` of a finished batch to
- * host. coeffs: 3 planes of i32, dense per group in decode order (group.rs:53). */
+ * host. coeffs: 3 planes of i32, dense per group in decode order (group.rs:53).
+ * xyb: the three padded XYB planes after dequant + IDCT; `stage` must be 0
+ * (any other value returns JXG_ERR_ARGUMENT). */
 int jxg_batch_read_coeffs(void* batch, uint32_t f, int32_t* out, size_t out_len);
 int jxg_batch_read_xyb(void* batch, uint32_t f, int stage, float* out, size_t out_len);
 
@@ -197,7 +194,8 @@ int jxg_batch_read_xyb(void* batch, uint32_t f, int stage, float* out, size_t ou
 int jxg_batch_set_deferred_copy(void* batch, int threads);
 
 /* Debug/parity: 0 = run everything (default), 1 = stop after the entropy kernel,
- * 2 = stop after dequant+IDCT (planes readable with stage 0). */
+ * 2 = stop after dequant+IDCT (planes readable with jxg_batch_read_xyb stage 0).
+ * Any other value returns JXG_ERR_ARGUMENT. */
 int jxg_batch_set_debug_stop(void* batch, int stage);
 
 /* Per-stage device timing with CUDA events on the launching stream (bench.py roofline):

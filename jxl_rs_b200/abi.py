@@ -69,7 +69,7 @@ EXPORTS = [
     "jxg_init", "jxg_shutdown", "jxg_batch_begin", "jxg_batch_add_frame", "jxg_batch_run", "jxg_batch_wait",
     "jxg_batch_rerun_device", "jxg_batch_end", "jxg_batch_read_coeffs", "jxg_batch_read_xyb",
     "jxg_batch_set_debug_stop", "jxg_batch_set_profile", "jxg_batch_stage_times", "jxg_batch_stage_marks", "jxg_batch_stats", "jxg_parse_file", "jxg_parse_file_mt", "jxg_parsed_free", "jxg_parsed_desc",
-    "jxg_batch_add_parsed", "jxg_batch_set_deferred_copy", "jxg_last_error", "jxg_device_pci_bus_id", "jxg_device_streams",
+    "jxg_batch_add_parsed", "jxg_batch_set_deferred_copy", "jxg_last_error", "jxg_device_pci_bus_id",
     "jxg_modular_parse_file", "jxg_modular_parsed_free", "jxg_modular_batch_begin", "jxg_modular_batch_add",
     "jxg_modular_batch_set_lanes", "jxg_modular_batch_run", "jxg_modular_batch_wait", "jxg_modular_batch_rerun_device",
     "jxg_modular_batch_read_planes", "jxg_modular_batch_stats", "jxg_modular_batch_end", "jxg_modular_walk_table",
@@ -97,7 +97,6 @@ def load_library():
     lib.jxg_last_error.restype = C.c_char_p
     lib.jxg_init.argtypes = [C.c_int, C.POINTER(vp)]
     lib.jxg_device_pci_bus_id.argtypes = [C.c_int, C.c_char_p, C.c_int]
-    lib.jxg_device_streams.argtypes = [C.c_int, C.POINTER(vp), C.POINTER(vp)]
     lib.jxg_shutdown.argtypes = [vp]
     lib.jxg_shutdown.restype = None
     lib.jxg_batch_begin.argtypes = [vp, C.c_uint32, C.POINTER(vp)]

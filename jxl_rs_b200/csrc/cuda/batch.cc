@@ -5,15 +5,11 @@
 
 #include <algorithm>
 #include <atomic>
-#include <thread>
 #include <chrono>
 #include <cmath>
 #include <cstdio>
 #include <cstring>
 #include <memory>
-#include <condition_variable>
-#include <deque>
-#include <functional>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -31,70 +27,23 @@ namespace detail {
 thread_local std::string g_error;
 std::atomic<int> g_live_contexts[64];  // per device: contexts between jxg_init and jxg_shutdown
 
-DeviceStreams device_streams(int device) {
+cudaStream_t device_d2h_stream(int device) {
   static std::mutex mu;
-  static DeviceStreams table[64];
+  static cudaStream_t table[64];
   std::lock_guard<std::mutex> lk(mu);
-  if (device < 0 || device >= 64) return DeviceStreams{};
-  DeviceStreams& d = table[device];
-  if (!d.entropy) {
+  if (device < 0 || device >= 64) return nullptr;
+  cudaStream_t& s = table[device];
+  if (!s) {
     cudaSetDevice(device);
-    if (cudaStreamCreateWithFlags(&d.entropy, cudaStreamNonBlocking) != cudaSuccess ||
-        cudaStreamCreateWithFlags(&d.post, cudaStreamNonBlocking) != cudaSuccess ||
-        cudaStreamCreateWithFlags(&d.d2h, cudaStreamNonBlocking) != cudaSuccess)
-      d = DeviceStreams{};
+    if (cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking) != cudaSuccess) s = nullptr;
   }
-  return d;
+  return s;
 }
 }
 }  // namespace jxgpu
 using namespace jxgpu::detail;
 
 namespace {
-
-// Host-ordered output copies (JXG_D2H_HOST_ORDERED=1): one thread per process takes the batches in launch order, waits on
-// the HOST for each frame range's filter launch (cudaEventSynchronize on a blocking-sync event) and only then enqueues that
-// range's D2H copies on the device's first-in-first-out copy stream. The copy stream then never holds a semaphore wait: a
-// stream parked on cudaStreamWaitEvent for tens of milliseconds (the next batch's filters) keeps the GPU's channel
-// scheduler from starting newly submitted streams - the first event of a new batch's stream was stamped 60 - 80 ms after
-// its submission, exactly when the output copies of the batch three launches earlier ended
-// (profiles/r02r_e2e_host_clock.log).
-class Copier {
- public:
-  static Copier& get() {
-    // never destroyed: its thread waits on the condition variable for the life of the process, and destroying a condition
-    // variable with a waiter blocks (glibc) - a static instance would hang every process at exit
-    static Copier* c = new Copier;
-    return *c;
-  }
-  void push(std::function<void()> job) {
-    std::lock_guard<std::mutex> lk(mu_);
-    if (!started_) {
-      started_ = true;
-      std::thread([this] { run(); }).detach();
-    }
-    q_.push_back(std::move(job));
-    cv_.notify_one();
-  }
-
- private:
-  void run() {
-    for (;;) {
-      std::function<void()> job;
-      {
-        std::unique_lock<std::mutex> lk(mu_);
-        cv_.wait(lk, [&] { return !q_.empty(); });
-        job = std::move(q_.front());
-        q_.pop_front();
-      }
-      job();
-    }
-  }
-  std::mutex mu_;
-  std::condition_variable cv_;
-  std::deque<std::function<void()>> q_;
-  bool started_ = false;
-};
 
 struct FrameOut {
   void* user_ptr;
@@ -111,9 +60,8 @@ struct Batch {
   Context* ctx;
   PinnedArena& blob;
   explicit Batch(Context* c)
-      : ctx(c), blob(c->blob), d_blob(c->d_blob), d_frames(c->d_frames), d_sections(c->d_sections), d_streams(c->d_streams), d_streams_lean(c->d_streams_lean), d_lean_cta(c->d_lean_cta), d_streams_fast(c->d_streams_fast), d_streams_slow(c->d_streams_slow),
-        d_nz_base(c->d_nz_base), d_tiles(c->d_tiles), d_ftiles(c->d_ftiles), d_coeffs(c->d_coeffs), d_block_off(c->d_block_off), d_nz(c->d_nz),
-        d_planes_a(c->d_planes_a), d_planes_b(c->d_planes_b), d_status(c->d_status), d_out(c->d_out) {}
+      : ctx(c), blob(c->blob), d_blob(c->d_blob), d_coeffs(c->d_coeffs), d_block_off(c->d_block_off), d_nz(c->d_nz),
+        d_planes_a(c->d_planes_a), d_status(c->d_status), d_out(c->d_out) {}
   std::vector<FrameDev> frames;
   std::vector<SectionDev> sections;
   std::vector<StreamDev> streams, streams_lean, streams_fast, streams_slow;
@@ -123,43 +71,25 @@ struct Batch {
   std::vector<uint32_t> lean_cta_first;
   std::vector<uint2> lean_warps;  // per warp of k_entropy_lean: first stream (relative to its frame's list), lanes
   std::vector<uint64_t> nz_base;
-  std::vector<uint32_t> tile_prefix{0};
   std::vector<uint32_t> fused_prefix{0};
   std::vector<FrameOut> outs;
   uint64_t total_groups = 0, total_blocks = 0, total_plane_floats = 0, nz_bytes = 0, out_bytes = 0, orient_bytes = 0;
   uint32_t lz_windows = 0;
-  uint32_t max_epf = 0;
   uint32_t filter_cfg_mask = 0;  // bit (gab * 4 + min(epf_iters, 3))
-  bool any_gab = false;
   int debug_stop = 0;
   // device
-  DevBuf &d_blob, &d_frames, &d_sections, &d_streams, &d_streams_lean, &d_lean_cta, &d_streams_fast, &d_streams_slow, &d_nz_base, &d_tiles, &d_ftiles, &d_coeffs, &d_block_off, &d_nz, &d_planes_a,
-      &d_planes_b, &d_status, &d_out;
+  DevBuf &d_blob, &d_coeffs, &d_block_off, &d_nz, &d_planes_a, &d_status, &d_out;
   bool uploaded = false;
   // byte offsets of the batch tables inside the blob (they ride on the one pinned H2D copy: a cudaMemcpyAsync from
   // pageable std::vector storage blocks the calling thread until earlier device work drains — 100+ ms with other
   // batches in flight, profiles/r02c_e2e_trace.log)
   struct {
     uint64_t frames = 0, sections = 0, streams = 0, lean_cta = 0, lean_warp = 0, streams_lean = 0, streams_fast = 0, streams_slow = 0,
-             nz_base = 0, tiles = 0, ftiles = 0;
+             nz_base = 0, ftiles = 0;
   } tab;
-  const float* final_planes = nullptr;
   int32_t* status_host = nullptr;  // pinned (context-owned): a D2H copy into pageable memory would block jxg_batch_run
   size_t status_n = 0;
-  cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_handoff = nullptr;
-  bool copies_on_copy_stream = false;  // last run: the D2H copies went to a copy stream (`copy_stream`), not the launching one
-  cudaStream_t copy_stream = nullptr;  // the device's shared D2H stream (default) or the context's own (JXG_D2H_SHARED=0)
-  // host-ordered copies: set by the copier thread once every copy and ev1 are enqueued (wait / end block on it first)
-  std::mutex copier_mu;
-  std::condition_variable copier_cv;
-  bool copier_pending = false;
-  bool host_ordered = false;  // this run's copies are enqueued by the copier thread
-  uint32_t host_ranges = 0;
-  int copier_error = 0;
-  void copier_wait() {
-    std::unique_lock<std::mutex> lk(copier_mu);
-    copier_cv.wait(lk, [&] { return !copier_pending; });
-  }
+  cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   cudaStream_t last_stream = nullptr;  // stream of the last run / rerun (the context's or the caller's)
   bool profile = false;
   cudaEvent_t stage_ev[kNumStages + 1] = {nullptr};
@@ -254,15 +184,6 @@ int jxg_device_pci_bus_id(int device, char* buf, int len) {
   return JXG_OK;
 }
 
-// The device's stage streams (see DeviceStreams), for hosts that want to bracket batches with their own events.
-int jxg_device_streams(int device, void** entropy_stream, void** post_stream) {
-  const DeviceStreams ds = device_streams(device);
-  if (!ds.entropy) return set_error(JXG_ERR_CUDA, "cannot create the device's stage streams");
-  if (entropy_stream) *entropy_stream = ds.entropy;
-  if (post_stream) *post_stream = ds.post;
-  return JXG_OK;
-}
-
 int jxg_init(int device, void** out_ctx) {
   if (!out_ctx) return JXG_ERR_ARGUMENT;
   int n = 0;
@@ -273,7 +194,8 @@ int jxg_init(int device, void** out_ctx) {
   auto ctx = std::make_unique<Context>();
   ctx->device = device;
   CUDA_TRY(cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
-  CUDA_TRY(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
+  ctx->d2h_stream = device_d2h_stream(device);
+  if (!ctx->d2h_stream) return set_error(JXG_ERR_CUDA, "cannot create the device's D2H stream");
   for (auto& e : ctx->range_done) CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming | cudaEventBlockingSync));
   CUDA_TRY(cudaEventCreateWithFlags(&ctx->copy_done, cudaEventDisableTiming | cudaEventBlockingSync));
   // constant tables
@@ -320,7 +242,6 @@ void jxg_shutdown(void* c) {
   if (!ctx) return;
   cudaSetDevice(ctx->device);
   if (ctx->stream) cudaStreamDestroy(ctx->stream);
-  if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
   for (auto& e : ctx->range_done)
     if (e) cudaEventDestroy(e);
   if (ctx->copy_done) cudaEventDestroy(ctx->copy_done);
@@ -344,11 +265,6 @@ int jxg_batch_begin(void* c, uint32_t n_frames_hint, void** out_batch) {
     cudaEventDestroy(b->ev0);
     return set_error(JXG_ERR_CUDA, std::string("cudaEventCreate: ") + cudaGetErrorString(e));
   }
-  if (cudaError_t e = cudaEventCreateWithFlags(&b->ev_handoff, cudaEventDisableTiming); e != cudaSuccess) {
-    cudaEventDestroy(b->ev0);
-    cudaEventDestroy(b->ev1);
-    return set_error(JXG_ERR_CUDA, std::string("cudaEventCreate: ") + cudaGetErrorString(e));
-  }
   cx->batch_live = true;  // only once nothing can fail any more
   *out_batch = b.release();
   return JXG_OK;
@@ -358,11 +274,9 @@ void jxg_batch_end(void* bp) {
   Batch* b = static_cast<Batch*>(bp);
   if (!b) return;
   cudaSetDevice(b->ctx->device);
-  b->copier_wait();
   if (b->uploaded && b->ev1) cudaEventSynchronize(b->ev1);
   if (b->ev0) cudaEventDestroy(b->ev0);
   if (b->ev1) cudaEventDestroy(b->ev1);
-  if (b->ev_handoff) cudaEventDestroy(b->ev_handoff);
   for (auto& e : b->stage_ev)
     if (e) cudaEventDestroy(e);
   b->ctx->batch_live = false;
@@ -382,7 +296,6 @@ int jxg_batch_set_profile(void* bp, int on) {
 int jxg_batch_stage_times(void* bp, float* ms, int n) {
   Batch* b = static_cast<Batch*>(bp);
   if (!b || !ms || n < kNumStages || !b->profile) return JXG_ERR_ARGUMENT;
-  b->copier_wait();
   CUDA_TRY(cudaEventSynchronize(b->ev1));
   for (int i = 0; i < kNumStages; i++) {
     ms[i] = 0.0f;
@@ -404,7 +317,6 @@ int jxg_batch_stage_marks(void* bp, float* ms, int n) {
     CUDA_TRY(cudaEventRecord(ref, 0));
     CUDA_TRY(cudaEventSynchronize(ref));
   }
-  b->copier_wait();
   CUDA_TRY(cudaEventSynchronize(b->ev1));
   for (int i = 0; i <= kNumStages; i++)
     if (cudaEventElapsedTime(&ms[i], ref, b->stage_ev[i]) != cudaSuccess) ms[i] = 0.0f;
@@ -428,7 +340,10 @@ int jxg_batch_set_deferred_copy(void* bp, int threads) {
 }
 
 int jxg_batch_set_debug_stop(void* bp, int stage) {
-  static_cast<Batch*>(bp)->debug_stop = stage;
+  Batch* b = static_cast<Batch*>(bp);
+  if (!b) return JXG_ERR_ARGUMENT;
+  if (stage < 0 || stage > 2) return set_error(JXG_ERR_ARGUMENT, "debug stop must be 0, 1 or 2");
+  b->debug_stop = stage;
   return JXG_OK;
 }
 
@@ -625,11 +540,7 @@ static int add_frame_impl(void* bp, const JxgFrameDesc* d, const uint8_t* hf_byt
     F.tf_hlg_exp = std::fabs(e) < 0.1f ? 0.0f : e;
   }
   F.tf_pq_mul = d->intensity_target * (1.0f / 10000.0f);
-  b->max_epf = std::max(b->max_epf, d->epf_iters);
-  b->any_gab = b->any_gab || d->gab;
   b->filter_cfg_mask |= 1u << ((d->gab ? 4 : 0) + std::min<uint32_t>(d->epf_iters, 3));
-  uint32_t tiles = ((F.width + 31) / 32) * ((F.height + 7) / 8);
-  b->tile_prefix.push_back(b->tile_prefix.back() + tiles);
   b->fused_prefix.push_back(b->fused_prefix.back() + ((F.width + kFusedTileW - 1) / kFusedTileW) * ((F.height + kFusedTileH - 1) / kFusedTileH));
   b->frames.push_back(F);
   return JXG_OK;
@@ -646,23 +557,15 @@ int jxg_batch_add_frame(void* bp, const JxgFrameDesc* d, const uint8_t* hf_bytes
 // that order (longest-processing-time rule), streams beyond the initial assignment are queued and pulled by whichever
 // lane finishes first. All CTAs of one frame stay on that frame so that its tables stay in L1 / shared memory.
 // Measured on B200 (64 x 4K, profiles/r02_entropy_schedule.md): every stream on a lane of its own from the start, four
-// lanes to a warp, is the fastest (33.1 ms); giving the longest streams warps of their own (`solo` / `duo` thresholds
-// as fractions of the frame's longest stream) is slower (38.6 - 41.4 ms) because a lone lane still costs a full warp's
-// issue slots, and so are fewer lanes with queued streams (43.9 ms at 2.5 streams per lane) and 8 lanes per warp (40.2).
-// The thresholds stay as experiment knobs (JXG_ENTROPY_SOLO / _DUO / _PER_LANE / _S).
+// lanes to a warp, is the fastest (33.1 ms); giving the longest streams warps of their own is slower (38.6 - 41.4 ms)
+// because a lone lane still costs a full warp's issue slots, and so are fewer lanes with queued streams (43.9 ms at 2.5
+// streams per lane) and 8 lanes per warp (40.2). Those alternatives were removed.
 static void schedule_lean(Batch* b) {
   if (b->streams_lean.empty() || b->lean_ctas) return;
   auto len_of = [&](const StreamDev& sd) { return b->sections[b->frames[sd.frame].section_base + sd.group].len; };
   std::stable_sort(b->streams_lean.begin(), b->streams_lean.end(), [&](const StreamDev& x, const StreamDev& y) {
     return x.frame != y.frame ? x.frame < y.frame : len_of(x) > len_of(y);
   });
-  auto knob = [](const char* name, float dflt) {
-    const char* e = getenv(name);
-    return e ? float(atof(e)) : dflt;
-  };
-  float solo = knob("JXG_ENTROPY_SOLO", 1.1f), duo = knob("JXG_ENTROPY_DUO", 1.1f);
-  // streams per packed lane (initial stream + queued ones): 1 = every stream starts at once
-  float per_lane = std::max(1.0f, knob("JXG_ENTROPY_PER_LANE", 1.0f));
   const size_t nf = b->frames.size();
   for (auto& F : b->frames) F.lean_first = F.lean_count = F.lean_cta_first = F.lean_ctas = F.lean_lanes = 0;
   for (size_t i = 0; i < b->streams_lean.size();) {
@@ -682,11 +585,7 @@ static void schedule_lean(Batch* b) {
   // profiles/r02k_entropy_lanes.log). Three or more live contexts on the device are taken as "batches share the SMs".
   uint32_t S = 4;
   if (g_live_contexts[b->ctx->device & 63].load() >= 3 && b->streams_lean.size() >= 2048) S = 8;
-  const char* s_env = getenv("JXG_ENTROPY_S");  // pins the lanes per warp (experiments)
-  if (s_env) S = uint32_t(atoi(s_env));
-  S = S <= 1 ? 1 : (S <= 2 ? 2 : (S <= 4 ? 4 : (S <= 8 ? 8 : (S <= 16 ? 16 : 32))));
-  // lanes actually used per packed warp (<= S, the kernel's compile-time capacity): 3 is a legal in-between
-  uint32_t L = std::min<uint32_t>(S, std::max<uint32_t>(1, uint32_t(knob("JXG_ENTROPY_LANES", float(S)))));
+  float per_lane = 1.0f;  // streams per lane (initial stream + queued ones): 1 = every stream starts at once
   std::vector<uint2> warps;
   for (int attempt = 0; attempt < 12; attempt++) {
     warps.clear();
@@ -696,38 +595,19 @@ static void schedule_lean(Batch* b) {
       F.lean_cta_first = ctas;
       F.lean_ctas = F.lean_lanes = 0;
       if (!F.lean_count) continue;
-      const float longest = float(len_of(b->streams_lean[F.lean_first])) + 64.0f;
-      uint32_t n_solo = 0, n_duo = 0;
-      for (uint32_t i = 0; i < F.lean_count; i++) {
-        const float l = float(len_of(b->streams_lean[F.lean_first + i])) + 64.0f;
-        if (S > 1 && l > solo * longest) n_solo++;
-        else if (S > 2 && l > duo * longest) n_duo++;
-        else break;
-      }
-      n_duo &= ~1u;
-      const uint32_t rest = F.lean_count - n_solo - n_duo;
-      uint32_t packed = uint32_t(std::ceil(float(rest) / per_lane));  // lanes of the S-wide warps
-      packed = std::min(rest, (packed + L - 1) / L * L);
+      uint32_t lanes = uint32_t(std::ceil(float(F.lean_count) / per_lane));
+      lanes = std::min(F.lean_count, (lanes + S - 1) / S * S);
       const size_t w0 = warps.size();
-      uint32_t pos = 0;
-      for (uint32_t i = 0; i < n_solo; i++) warps.push_back(make_uint2(pos++, 1));
-      for (uint32_t i = 0; i < n_duo; i += 2, pos += 2) warps.push_back(make_uint2(pos, 2));
-      for (uint32_t i = 0; i < packed; i += L) {
-        const uint32_t n = std::min(L, packed - i);
-        warps.push_back(make_uint2(pos, n));
-        pos += n;
-      }
+      for (uint32_t pos = 0; pos < lanes; pos += S) warps.push_back(make_uint2(pos, std::min(S, lanes - pos)));
       while ((warps.size() - w0) % 4) warps.push_back(make_uint2(F.lean_count, 0));  // idle warps of the frame's last CTA
-      F.lean_lanes = pos;
+      F.lean_lanes = lanes;
       F.lean_ctas = uint32_t(warps.size() - w0) / 4;
       ctas += F.lean_ctas;
     }
     b->lean_ctas = ctas;
     if (ctas <= max_ctas) break;
-    // denser: first fewer privileged warps, then 8 lanes per warp, then more streams per packed lane
-    if (solo < 0.95f) solo = std::min(0.95f, solo + 0.1f), duo = std::min(0.9f, duo + 0.1f);
-    else if (L < S) L = S;
-    else if (S < 8 && !s_env) S = L = 8;
+    // denser: first 8 lanes per warp, then more streams per lane
+    if (S < 8) S = 8;
     else per_lane *= 1.3f;
   }
   b->lean_S = S;
@@ -752,14 +632,12 @@ static BatchDev make_batch_dev(Batch* b) {
   B.streams_slow = reinterpret_cast<const StreamDev*>(tab(b->tab.streams_slow));
   B.num_fast = uint32_t(b->streams_fast.size());
   B.num_slow = uint32_t(b->streams_slow.size());
-  B.reg_idct32 = (getenv("JXG_REG_IDCT32") && atoi(getenv("JXG_REG_IDCT32"))) ? 1u : 0u;
   B.nzlist = static_cast<uint32_t*>(b->d_coeffs.p);  // the pool that held the dense coefficients now holds the lists
   B.block_off = static_cast<uint32_t*>(b->d_block_off.p);
   B.lzwin = static_cast<uint32_t*>(b->ctx->d_lzwin.p);
   B.nz = static_cast<uint8_t*>(b->d_nz.p);
   B.nz_base = reinterpret_cast<uint64_t*>(const_cast<uint8_t*>(tab(b->tab.nz_base)));
   B.planes_a = static_cast<float*>(b->d_planes_a.p);
-  B.planes_b = static_cast<float*>(b->d_planes_b.p);
   B.status = static_cast<int32_t*>(b->d_status.p);
   B.queue = reinterpret_cast<uint32_t*>(B.status + b->streams.size());
   B.lean_cta_first = reinterpret_cast<const uint32_t*>(tab(b->tab.lean_cta));
@@ -773,43 +651,18 @@ static BatchDev make_batch_dev(Batch* b) {
   return B;
 }
 
-// se: stream of the upload, block plan and entropy kernels; s: stream of everything after them (== se when the caller
-// brought its own stream).
-static int launch(Batch* b, cudaStream_t se, cudaStream_t s, bool copy_to_host) {
+// Enqueues one run of the batch on `s`. With copy_to_host, the host outputs go back on the device's D2H stream: each of
+// up to kMaxRanges frame ranges is copied as soon as its filter launch ends, while the next range is being filtered.
+static int launch(Batch* b, cudaStream_t s, bool copy_to_host) {
   const BatchDev B = make_batch_dev(b);
-  auto tab = [&](uint64_t off) { return static_cast<const uint8_t*>(b->d_blob.p) + off; };
-  size_t coeff_bytes = 0;
   cudaEvent_t* ev = b->profile ? b->stage_ev : nullptr;
-  b->launches = uint64_t(launch_pipeline(B, reinterpret_cast<const uint32_t*>(tab(b->tab.tiles)), b->tile_prefix.back(), b->max_epf,
-                                         b->any_gab, se, coeff_bytes, &b->final_planes, b->debug_stop, ev,
-                                         reinterpret_cast<const uint32_t*>(tab(b->tab.ftiles)), b->fused_prefix.back(),
-                                         b->filter_cfg_mask, b->lean_all_420, b->lean_S, b->lean_ctas,
-                                         b->lean_ctx_smem && !(getenv("JXG_LEAN_CTX_SMEM") && atoi(getenv("JXG_LEAN_CTX_SMEM")) == 0),
-                                         s, b->ev_handoff));
-  if (b->debug_stop == 1 && s != se) {  // stopped after the entropy stage: the post stream still has to cover it
-    cudaEventRecord(b->ev_handoff, se);
-    cudaStreamWaitEvent(s, b->ev_handoff, 0);
-  }
+  b->launches = uint64_t(launch_pipeline(B, s, b->debug_stop, ev, b->lean_all_420, b->lean_S, b->lean_ctas, b->lean_ctx_smem));
   if (b->debug_stop == 0) {
-    // Fused filter + colour + store, launched per range of frames; each finished range is copied to the host
-    // on the copy stream while the next range is being filtered.
+    // Fused filter + colour + store, launched per range of frames.
     Context* cx = b->ctx;
     const uint32_t nf = uint32_t(b->frames.size());
-    // D2H of host outputs: JXG_D2H_RANGES = r > 0 copies each of r frame ranges on the copy stream as soon as its filter
-    // launch ends (lowest latency for one batch alone); 0 = one filter launch, then all copies on the launching stream
-    // (no cross-stream events: with several batches in flight on several contexts the copies of batch k overlap the
-    // kernels of batch k + 1 anyway).
-    static const int d2h_ranges = getenv("JXG_D2H_RANGES") ? atoi(getenv("JXG_D2H_RANGES")) : int(Context::kMaxRanges);
-    const bool same_stream = copy_to_host && d2h_ranges <= 0;
-    const uint32_t nr = (copy_to_host && !same_stream) ? std::min<uint32_t>(std::min<uint32_t>(uint32_t(d2h_ranges), Context::kMaxRanges), nf) : 1;
-    static const bool shared_d2h = !(getenv("JXG_D2H_SHARED") && atoi(getenv("JXG_D2H_SHARED")) == 0);
-    static const bool host_ordered_env = getenv("JXG_D2H_HOST_ORDERED") && atoi(getenv("JXG_D2H_HOST_ORDERED")) != 0;
-    b->host_ordered = host_ordered_env && copy_to_host && !same_stream;
-    b->host_ranges = nr;
-    const DeviceStreams ds = device_streams(cx->device);
-    b->copy_stream = (shared_d2h && ds.d2h) ? ds.d2h : cx->copy_stream;
-    cudaStream_t cs = same_stream ? s : b->copy_stream;
-    const uint32_t* fp = reinterpret_cast<const uint32_t*>(tab(b->tab.ftiles));
+    const uint32_t nr = copy_to_host ? std::min<uint32_t>(Context::kMaxRanges, nf) : 1;
+    const uint32_t* fp = reinterpret_cast<const uint32_t*>(static_cast<const uint8_t*>(b->d_blob.p) + b->tab.ftiles);
     if (ev) {
       for (int i = 4; i <= 6; i++) cudaEventRecord(ev[i], s);
     }
@@ -826,15 +679,13 @@ static int launch(Batch* b, cudaStream_t se, cudaStream_t s, bool copy_to_host) 
         b->launches++;
       }
       if (copy_to_host) {
-        if (!same_stream) {
-          CUDA_TRY(cudaEventRecord(cx->range_done[r], s));
-          if (b->host_ordered) continue;  // the copier thread waits for the event and enqueues this range's copies
-          CUDA_TRY(cudaStreamWaitEvent(cs, cx->range_done[r], 0));
-        }
+        CUDA_TRY(cudaEventRecord(cx->range_done[r], s));
+        CUDA_TRY(cudaStreamWaitEvent(cx->d2h_stream, cx->range_done[r], 0));
         for (uint32_t f = f0; f < f1; f++) {
           const FrameOut& fo = b->outs[f];
           if (fo.is_device) continue;
-          CUDA_TRY(cudaMemcpyAsync(fo.user_ptr, static_cast<uint8_t*>(b->d_out.p) + fo.dev_off, fo.copy_bytes, cudaMemcpyDeviceToHost, cs));
+          CUDA_TRY(cudaMemcpyAsync(fo.user_ptr, static_cast<uint8_t*>(b->d_out.p) + fo.dev_off, fo.copy_bytes, cudaMemcpyDeviceToHost,
+                                   cx->d2h_stream));
           b->d2h += fo.copy_bytes;
         }
       }
@@ -843,7 +694,6 @@ static int launch(Batch* b, cudaStream_t se, cudaStream_t s, bool copy_to_host) 
       cudaEventRecord(ev[7], s);
       cudaEventRecord(ev[8], s);
     }
-    b->copies_on_copy_stream = copy_to_host && !same_stream;
   }
   CUDA_TRY(cudaGetLastError());
   return 0;
@@ -878,12 +728,7 @@ int jxg_batch_run(void* bp, void* cuda_stream) {
   if (!b || b->frames.empty()) return JXG_ERR_ARGUMENT;
   RunTrace trace;
   CUDA_TRY(cudaSetDevice(b->ctx->device));
-  // the caller's stream for everything, or the device's stage streams (see DeviceStreams)
-  const DeviceStreams ds = device_streams(b->ctx->device);
-  static const bool staged = getenv("JXG_STAGE_STREAMS") && atoi(getenv("JXG_STAGE_STREAMS")) != 0;
-  const bool use_pair = !cuda_stream && staged && ds.entropy;
-  cudaStream_t se = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : (use_pair ? ds.entropy : b->ctx->stream);
-  cudaStream_t s = cuda_stream ? se : (use_pair ? ds.post : b->ctx->stream);
+  cudaStream_t s = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : b->ctx->stream;
   b->last_stream = s;
   b->h2d = b->d2h = 0;
   schedule_lean(b);
@@ -894,7 +739,6 @@ int jxg_batch_run(void* bp, void* cuda_stream) {
   if (int r = b->ctx->d_lzwin.ensure(std::max<size_t>(size_t(b->lz_windows) * kLzWindow * 4, 16))) return r;
   if (int r = b->d_nz.ensure(b->nz_bytes)) return r;
   if (int r = b->d_planes_a.ensure(b->total_plane_floats * 4)) return r;
-  if (int r = b->d_planes_b.ensure(b->total_plane_floats * 4)) return r;
   if (int r = b->d_status.ensure((b->streams.size() + b->frames.size() + 4) * 4)) return r;
   if (int r = b->d_out.ensure(std::max<size_t>(b->out_bytes, 16))) return r;
   if (int r = b->ctx->d_lean_desc.ensure(std::max<size_t>(b->streams.size() * 1024 * 16, 16))) return r;
@@ -930,82 +774,29 @@ int jxg_batch_run(void* bp, void* cuda_stream) {
               put(b->streams_fast.data(), b->streams_fast.size() * sizeof(StreamDev), b->tab.streams_fast) &&
               put(b->streams_slow.data(), b->streams_slow.size() * sizeof(StreamDev), b->tab.streams_slow) &&
               put(b->nz_base.data(), b->nz_base.size() * 8, b->tab.nz_base) &&
-              put(b->tile_prefix.data(), b->tile_prefix.size() * 4, b->tab.tiles) &&
               put(b->fused_prefix.data(), b->fused_prefix.size() * 4, b->tab.ftiles);
     if (!ok) return set_error(JXG_ERR_CUDA, "pinned staging allocation failed");
   }
-  if (!b->blob.reserve(b->blob.size + 16)) return set_error(JXG_ERR_CUDA, "pinned staging allocation failed");  // k_upload reads whole 16-byte words
   if (int r = b->d_blob.ensure(b->blob.size + 64)) return r;
   trace.mark("alloc");
   b->blob.flush();
   trace.mark("flush");
-  if (use_pair) {
-    // the upload rides on the context's own stream so that it overlaps the entropy kernel of the batch before;
-    // the entropy stream picks it up through the hand-off event (free again once launch() re-records it)
-    CUDA_TRY(cudaEventRecord(b->ev0, b->ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(b->d_blob.p, b->blob.p, b->blob.size, cudaMemcpyHostToDevice, b->ctx->stream));
-    CUDA_TRY(cudaEventRecord(b->ev_handoff, b->ctx->stream));
-    CUDA_TRY(cudaStreamWaitEvent(se, b->ev_handoff, 0));
-  } else {
-    CUDA_TRY(cudaEventRecord(b->ev0, se));
-    // JXG_UPLOAD_KERNEL=1: the SMs fetch the blob from pinned host memory instead of a copy engine. With several batches
-    // in flight the copy engine's queue holds the D2H copies of older batches, and an H2D cudaMemcpyAsync submitted behind
-    // them does not start until that queue runs dry (profiles/r02m_e2e_fifo.log: the first event of a batch's stream is
-    // stamped when the D2H of the batch three launches earlier ends) - the new batch's kernels wait with it.
-    static const bool upload_kernel = getenv("JXG_UPLOAD_KERNEL") && atoi(getenv("JXG_UPLOAD_KERNEL")) != 0;
-    if (upload_kernel) launch_upload(b->blob.p, b->d_blob.p, b->blob.size, se);
-    else CUDA_TRY(cudaMemcpyAsync(b->d_blob.p, b->blob.p, b->blob.size, cudaMemcpyHostToDevice, se));
-  }
+  CUDA_TRY(cudaEventRecord(b->ev0, s));
+  CUDA_TRY(cudaMemcpyAsync(b->d_blob.p, b->blob.p, b->blob.size, cudaMemcpyHostToDevice, s));
   trace.mark("blob_h2d");
   b->h2d += b->blob.size;
   b->uploaded = true;
   trace.mark("uploads");
-  b->copies_on_copy_stream = false;
-  if (int r = launch(b, se, s, true)) return r;
+  if (int r = launch(b, s, true)) return r;
   trace.mark("launch");
   if (int r = copy_status(b, s)) return r;
-  // ev1 = everything of this batch done. The copy stream joins the post stream and carries ev1 when it holds the D2H
-  // copies: the post stream itself must not wait for them (the next batch's transforms follow on it).
-  if (b->copies_on_copy_stream && b->host_ordered) {
-    Context* cx = b->ctx;
-    CUDA_TRY(cudaEventRecord(cx->copy_done, s));  // behind the status words
-    {
-      std::lock_guard<std::mutex> lk(b->copier_mu);
-      b->copier_pending = true;
-      b->copier_error = 0;
-    }
-    Copier::get().push([b] {
-      Context* cx = b->ctx;
-      int err = 0;
-      auto chk = [&](cudaError_t e) {
-        if (e != cudaSuccess && !err) err = int(e);
-      };
-      chk(cudaSetDevice(cx->device));
-      const uint32_t nf = uint32_t(b->frames.size()), nr = b->host_ranges;
-      for (uint32_t r = 0; r < nr && !err; r++) {
-        chk(cudaEventSynchronize(cx->range_done[r]));  // host-side wait: nothing parks on the copy stream
-        const uint32_t f0 = uint32_t(uint64_t(nf) * r / nr), f1 = uint32_t(uint64_t(nf) * (r + 1) / nr);
-        for (uint32_t f = f0; f < f1 && !err; f++) {
-          const FrameOut& fo = b->outs[f];
-          if (fo.is_device) continue;
-          chk(cudaMemcpyAsync(fo.user_ptr, static_cast<uint8_t*>(b->d_out.p) + fo.dev_off, fo.copy_bytes, cudaMemcpyDeviceToHost,
-                              b->copy_stream));
-        }
-      }
-      chk(cudaEventSynchronize(cx->copy_done));
-      chk(cudaEventRecord(b->ev1, b->copy_stream));
-      std::lock_guard<std::mutex> lk(b->copier_mu);
-      b->copier_error = err;
-      b->copier_pending = false;
-      b->copier_cv.notify_all();
-    });
-    for (const FrameOut& fo : b->outs)
-      if (!fo.is_device) b->d2h += fo.copy_bytes;
-  } else if (b->copies_on_copy_stream) {
+  // ev1 = everything of this batch done. The D2H stream joins the launching stream and carries ev1 when it holds the
+  // output copies: the launching stream itself must not wait for them.
+  if (b->debug_stop == 0) {
     Context* cx = b->ctx;
     CUDA_TRY(cudaEventRecord(cx->copy_done, s));
-    CUDA_TRY(cudaStreamWaitEvent(b->copy_stream, cx->copy_done, 0));
-    CUDA_TRY(cudaEventRecord(b->ev1, b->copy_stream));
+    CUDA_TRY(cudaStreamWaitEvent(cx->d2h_stream, cx->copy_done, 0));
+    CUDA_TRY(cudaEventRecord(b->ev1, cx->d2h_stream));
   } else {
     CUDA_TRY(cudaEventRecord(b->ev1, s));
   }
@@ -1017,15 +808,11 @@ int jxg_batch_rerun_device(void* bp, void* cuda_stream) {
   Batch* b = static_cast<Batch*>(bp);
   if (!b || !b->uploaded) return set_error(JXG_ERR_ARGUMENT, "batch was never submitted");
   CUDA_TRY(cudaSetDevice(b->ctx->device));
-  const DeviceStreams ds = device_streams(b->ctx->device);
-  static const bool staged = getenv("JXG_STAGE_STREAMS") && atoi(getenv("JXG_STAGE_STREAMS")) != 0;
-  const bool use_pair = !cuda_stream && staged && ds.entropy;
-  cudaStream_t se = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : (use_pair ? ds.entropy : b->ctx->stream);
-  cudaStream_t s = cuda_stream ? se : (use_pair ? ds.post : b->ctx->stream);
+  cudaStream_t s = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : b->ctx->stream;
   b->last_stream = s;
-  CUDA_TRY(cudaStreamWaitEvent(se, b->ev1, 0));  // the previous run of this batch still owns its device buffers
-  CUDA_TRY(cudaEventRecord(b->ev0, se));
-  if (int r = launch(b, se, s, false)) return r;
+  CUDA_TRY(cudaStreamWaitEvent(s, b->ev1, 0));  // the previous run of this batch still owns its device buffers
+  CUDA_TRY(cudaEventRecord(b->ev0, s));
+  if (int r = launch(b, s, false)) return r;
   CUDA_TRY(cudaMemcpyAsync(b->status_host, b->d_status.p, b->status_n * 4, cudaMemcpyDeviceToHost, s));
   CUDA_TRY(cudaEventRecord(b->ev1, s));
   return JXG_OK;
@@ -1038,11 +825,9 @@ int jxg_batch_wait(void* bp, uint32_t* first_bad_frame, uint32_t* first_bad_grou
   {
     static const bool traced = getenv("JXG_TRACE_RUN") && atoi(getenv("JXG_TRACE_RUN")) != 0;
     const auto t0 = std::chrono::steady_clock::now();
-    b->copier_wait();  // host-ordered copies: ev1 exists only once the copier has enqueued everything
-    if (b->copier_error) return set_error(JXG_ERR_CUDA, std::string("output copy failed: ") + cudaGetErrorString(cudaError_t(b->copier_error)));
     const bool was_done = traced && cudaEventQuery(b->ev1) == cudaSuccess;
     CUDA_TRY(cudaEventSynchronize(b->ev1));  // recorded behind the status words and the D2H copies; no stream-wide wait:
-                                             // the stage streams carry later batches too
+                                             // the D2H stream carries later batches too
     if (traced)
       fprintf(stderr, "[jxg_batch_wait] done on entry %d, event wait %.1f ms\n", int(was_done),
               std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count());
@@ -1090,15 +875,13 @@ int jxg_batch_read_coeffs(void* bp, uint32_t f, int32_t* out, size_t out_len) {
 
 int jxg_batch_read_xyb(void* bp, uint32_t f, int stage, float* out, size_t out_len) {
   Batch* b = static_cast<Batch*>(bp);
-  if (!b || f >= b->frames.size() || !b->uploaded) return JXG_ERR_ARGUMENT;
+  if (!b || f >= b->frames.size() || !b->uploaded || stage != 0) return JXG_ERR_ARGUMENT;
   const FrameDev& F = b->frames[f];
   size_t n = 3 * F.plane_size;
   if (out_len < n) return JXG_ERR_ARGUMENT;
-  const float* src = stage == 0 ? static_cast<const float*>(b->d_planes_a.p) : b->final_planes;
-  if (!src) return JXG_ERR_ARGUMENT;
   CUDA_TRY(cudaSetDevice(b->ctx->device));
   CUDA_TRY(cudaStreamSynchronize(b->ctx->stream));
-  CUDA_TRY(cudaMemcpy(out, src + F.plane_base, n * 4, cudaMemcpyDeviceToHost));
+  CUDA_TRY(cudaMemcpy(out, static_cast<const float*>(b->d_planes_a.p) + F.plane_base, n * 4, cudaMemcpyDeviceToHost));
   return JXG_OK;
 }
 

@@ -108,26 +108,18 @@ struct PinnedArena {
   }
 };
 
-// Optional (JXG_STAGE_STREAMS=1): two streams per DEVICE shared by all its contexts — every batch runs its block plan and
-// entropy kernels on the entropy stream and its transforms, filters and stores on the post stream, so that at most one
-// kernel of each kind runs at a time. Measured slower than one stream per batch on B200 (53 - 56 against 44 - 50 ms per
-// 64-frame step, profiles/r02h_stage_stream_sweep.log): the entropy kernel parks ~30 K of an SM's 64 K registers for its
-// whole duration, so the transforms / filters beside it run at one CTA per SM, and nothing is gained over letting
-// batches overlap in the entropy kernel's tail. The default is one stream per batch.
-struct DeviceStreams {
-  cudaStream_t entropy = nullptr, post = nullptr;
-  // One D2H stream for all contexts of the device: output copies leave in launch order. With a copy stream per context
-  // the copies of all batches in flight share the host link evenly, so they all end together, all contexts come free
-  // together and the next batches start together: a convoy that leaves the SMs idle for the length of the D2H tail
-  // (profiles/r02l_e2e_convoy.log). First in, first out retires the oldest batch early and keeps the launches staggered.
-  cudaStream_t d2h = nullptr;
-};
-DeviceStreams device_streams(int device);  // created on first use
+// One D2H stream for all contexts of the device: output copies leave in launch order. With a copy stream per context
+// the copies of all batches in flight share the host link evenly, so they all end together, all contexts come free
+// together and the next batches start together: a convoy that leaves the SMs idle for the length of the D2H tail
+// (profiles/r02l_e2e_convoy.log). First in, first out retires the oldest batch early and keeps the launches staggered.
+// Created by the first jxg_init on the device; nullptr if that failed.
+cudaStream_t device_d2h_stream(int device);
 
 struct Context {
   int device = 0;
   cudaStream_t stream = nullptr;
-  cudaStream_t copy_stream = nullptr;  // D2H of finished frame ranges overlaps the filtering of later ranges
+  cudaStream_t d2h_stream = nullptr;  // device_d2h_stream (not owned): D2H of finished frame ranges overlaps the
+                                      // filtering of later ranges
   static constexpr int kMaxRanges = 8;
   cudaEvent_t range_done[kMaxRanges] = {nullptr}, copy_done = nullptr;
   DevBuf dequant_default, dequant_default_off, natural_orders, natural_order_off;
@@ -135,8 +127,7 @@ struct Context {
   // intermediates and the pinned staging arena survive jxg_batch_end so that a
   // steady-state decode loop does no cudaMalloc / cudaHostAlloc.
   PinnedArena blob;
-  DevBuf d_blob, d_frames, d_sections, d_streams, d_streams_lean, d_lean_cta, d_streams_fast, d_streams_slow, d_nz_base, d_tiles, d_ftiles, d_coeffs, d_block_off, d_nz, d_planes_a,
-      d_planes_b, d_status, d_out, d_lean_desc, d_lean_nblk, d_orient, d_lean_warp, d_big, d_lzwin;
+  DevBuf d_blob, d_coeffs, d_block_off, d_nz, d_planes_a, d_status, d_out, d_lean_desc, d_lean_nblk, d_orient, d_lzwin;
   bool batch_live = false;
   // pinned status readback buffer, owned by the context: cudaHostAlloc / cudaFreeHost synchronise the whole
   // device, so they must not happen per batch when batches of several contexts are in flight

@@ -112,14 +112,12 @@ struct BatchDev {
   const StreamDev* streams_fast;  // single-pass prefix-coded frames: k_entropy_fast
   const StreamDev* streams_slow;  // multi-pass frames: k_entropy
   uint32_t num_frames, num_streams, num_lean, num_fast, num_slow;
-  uint32_t reg_idct32;  // 1: rows of 32 coefficients also go through the register path (experiment knob)
   uint32_t* nzlist;     // [sections][kListStride]: list of section (pass * num_groups + group) of a frame, see above
   uint32_t* lzwin;      // [lz sections][kLzWindow] LZ77 windows (decode.rs:86-146), frames with has_lz only
   uint32_t* block_off;  // per 8x8 block: ordinal (raster order) of the varblock starting there within its group
   uint8_t* nz;          // [streams][passes][3][1024]
   uint64_t* nz_base;    // per stream offset into nz (bytes)
   float* planes_a;
-  float* planes_b;
   int32_t* status;      // per stream
   uint32_t* queue;      // [frames] work-queue cursors of the persistent entropy kernel
   const uint32_t* lean_cta_first;  // [frames] first CTA of each frame in k_entropy_lean's grid

@@ -232,7 +232,6 @@ void add_frame(ModularBatch* b, jxg::ModularFrameState* ms, void* out, size_t st
   uint32_t global_code = 0;
   uint64_t global_tree = 0;
   bool have_global = false;
-  static const bool walk_tables = !(getenv("JXG_MODULAR_WALK_TABLES") && atoi(getenv("JXG_MODULAR_WALK_TABLES")) == 0);
   std::map<WalkKey, WalkInfo> walk_cache;
   std::map<uint64_t, bool> inner_static;
   f.first_stream = uint32_t(b->streams.size());
@@ -275,7 +274,7 @@ void add_frame(ModularBatch* b, jxg::ModularFrameState* ms, void* out, size_t st
       rd.h = r.h;
       rd.walk = kWalkGeneric;
       rd.lut_off = 0;
-      if (walk_tables && r.w && r.h) {
+      if (r.w && r.h) {
         const uint32_t root = static_root(*tree, uint32_t(ri), st.stream_id);
         // channel / stream decisions below another split make the table specific to this channel of this stream
         auto is_it = inner_static.find(d.tree_off);

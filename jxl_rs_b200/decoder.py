@@ -110,7 +110,7 @@ class Batch:
                                                            row_stride, 1 if out_is_device else 0))
 
     def set_debug_stop(self, stage: int):
-        self._lib.jxg_batch_set_debug_stop(self._h, stage)
+        abi.check(self._lib, self._lib.jxg_batch_set_debug_stop(self._h, stage))
 
     STAGES = ["memset", "entropy", "dequant_idct", "gaborish", "epf0", "epf1", "epf2", "xyb_store"]
 
@@ -203,12 +203,9 @@ def decode_files(ctx: JxgContext, files, pixel_format: JxlPixelFormat = JxlPixel
 
 
 def device_streams(device: int = 0):
-    """(entropy stream, post stream) of the device as raw cudaStream_t values (jxg_device_streams): the optional stage
-    streams (JXG_STAGE_STREAMS=1); by default every batch runs on its context's own stream."""
-    lib = abi.load_library()
-    e, p = C.c_void_p(), C.c_void_p()
-    abi.check(lib, lib.jxg_device_streams(device, C.byref(e), C.byref(p)))
-    return e.value, p.value
+    """The per-device stage streams (JXG_STAGE_STREAMS) are gone: every batch runs on one stream, its context's or the
+    caller's. Callers of the old name get this error instead of an AttributeError."""
+    raise abi.JxgError(-2, "the stage-stream mode was removed; batches run on their context's stream or the caller's")
 
 
 def _parse_cpulist(text):
